@@ -28,14 +28,19 @@ import argparse
 import ctypes
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 os.environ.setdefault("SAILGPU_TIMING", "1")
+# the bench may run from a read-only tree: no bytecode caches there, neither here nor in the legs' subprocesses
+sys.dont_write_bytecode = True
+os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
 
 Q1_COLS = ["l_quantity", "l_extendedprice", "l_discount", "l_tax", "l_returnflag", "l_linestatus", "l_shipdate"]
 ALGO_BYTES_PER_ROW = 100      # 4 x Decimal128 + 2 x Utf8View + Date32  (SURVEY.md section 8d)
@@ -59,7 +64,42 @@ def parse_args():
     ap.add_argument("--skip-joins", action="store_true")
     ap.add_argument("--skip-suites", action="store_true", help="skip the 22-query TPC-H total and the ClickBench leg (N = 1)")
     ap.add_argument("--suite-sf", type=float, default=10.0, help="scale factor of the 22-query TPC-H leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the Q1 result of the last timed step as DIR/<column>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def private_jit_cache() -> tempfile.TemporaryDirectory:
+    """The library caches the kernels it specialises next to itself (sail_b200/_build/jit_cache) unless SAILGPU_JIT_CACHE
+    names another directory.  The bench writes nothing into its tree, so it points the library at a temporary copy of the
+    cache build() filled: the bench pipelines still find their kernels, and anything compiled at run time goes to the copy."""
+    tmp = tempfile.TemporaryDirectory(prefix="sailgpu_jit_")
+    seed = os.path.join(ROOT, "sail_b200", "_build", "jit_cache")
+    if os.path.isdir(seed):
+        shutil.copytree(seed, tmp.name, dirs_exist_ok=True)
+    os.environ["SAILGPU_JIT_CACHE"] = tmp.name
+    return tmp
+
+
+def dump_outputs(table, out_dir: str) -> None:
+    """One float64 array per result column, DIR/<column>.npy, rows in the order the caller received them: numbers and
+    decimals by value, strings as their UTF-8 bytes (one zero-padded row per value).  The inputs come from the seeded
+    generator, so two builds run with the same arguments can be compared array for array."""
+    import numpy as np
+    import pyarrow as pa
+    os.makedirs(out_dir, exist_ok=True)
+    for name, col in zip(table.column_names, table.columns):
+        vals = col.to_pylist()
+        if pa.types.is_string(col.type) or pa.types.is_large_string(col.type) or pa.types.is_string_view(col.type):
+            raw = [v.encode() for v in vals]
+            arr = np.zeros((len(raw), max([1] + [len(b) for b in raw])), dtype=np.float64)
+            for i, b in enumerate(raw):
+                arr[i, :len(b)] = list(b)
+        else:
+            arr = np.array([np.nan if v is None else float(v) for v in vals], dtype=np.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
 
 
 def host_cores() -> int:
@@ -620,6 +660,7 @@ def main():
         if rank != 0:
             return 0
         return run_reference(args)
+    jit_cache = private_jit_cache()      # noqa: F841 -- removed when main() returns
 
     import torch
     import torch.distributed as dist
@@ -711,6 +752,8 @@ def main():
                 check_result(acc["out"], want_rows)
     elif not args.skip_e2e:
         host_e2e = [g.host_table() for g in gens[: args.e2e_chunks]]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(acc["out"], args.dump_outputs)
     ms_per_step = ms / args.steps
     value = total_rows / (ms_per_step / 1e3)
     out = acc["out"]
